@@ -9,6 +9,10 @@ buffers (pinned H2D of z/pos/n_atoms and D2H of E,F inside the timed region ever
 
 `--impl reference` times the CPU oracle restatement of the reference path (the reference
 itself cannot be imported on this image: schnetpack/PyG/e3nn absent) on all host cores.
+
+`--dump-outputs DIR` writes the energies and forces of the last timed step as DIR/energy.npy and
+DIR/forces.npy (float32).  Inputs and weights are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 import argparse
 import json
@@ -86,6 +90,15 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+def dump_outputs(directory, energy, forces):
+    """What a caller of the timed path receives from one step: per-molecule energies [n_mol], per-atom forces [n_atoms, 3]."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, t in (("energy", energy), ("forces", forces)):
+        np.save(os.path.join(directory, name + ".npy"), t.detach().cpu().float().numpy())
 
 
 def build_model(kind, device):
@@ -235,7 +248,7 @@ def train_record(args, dev, rank, world, storage="f32"):
     torch.cuda.synchronize()
     if world > 1:
         torch.distributed.barrier()
-    steps = 6
+    steps = args.steps
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for k in range(steps):
@@ -277,8 +290,10 @@ def run_reference(args):
         oracle_pass(kind, ref, b, min(8, sample))
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        oracle_pass(kind, ref, b, sample)
+        out = oracle_pass(kind, ref, b, sample)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *out)
     val = args.steps * sample / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": "molecules/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -310,7 +325,10 @@ def main():
     ap.add_argument("--node", default="fused", choices=["fused", "unfused"], help="per-atom part of a layer: fused tcgen05 kernels (default) or one launch per op (round 1)")
     ap.add_argument("--skip-e2e", action="store_true", help="profiling runs only (ncu): device-resident leg only")
     ap.add_argument("--no-train", action="store_true", help="skip the training sub-record (BASELINE configs[2] shape)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the energies and forces of the last timed step to DIR/energy.npy, DIR/forces.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     global B_PER_GPU
     B_PER_GPU = args.batch
@@ -408,6 +426,8 @@ def main():
     for r_ in last:
         if r_ is not None:
             eng.raise_on_status(r_[2].cpu())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last[(args.steps - 1) % n_str][:2])
     e, f, st = step_dev(0)
     torch.cuda.synchronize()
     eng.raise_on_status(st.cpu())
@@ -468,7 +488,7 @@ def main():
     for k in range(3 * S2):
         step_e2e(k)
     barrier()
-    e2e_steps = max(12, args.steps // 2)
+    e2e_steps = args.steps
     ev0.record()
     for s_ in e2e_streams:
         s_.wait_event(ev0)

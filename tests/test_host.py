@@ -190,21 +190,22 @@ def test_b200_model_yamls_instantiate():
     pyg_keys = ["_target_", "model_name", "net", "optimizer", "lr_scheduler", "losses", "loss_coefs", "metric"]
     top = {"painn-b200.yaml": spk_keys, "schnet-b200.yaml": spk_keys, "painn-oc-b200.yaml": [k if k != "net" else "model" for k in pyg_keys],
            "qhnet-b200.yaml": pyg_keys + ["ema"], "gemnet-oc-b200.yaml": pyg_keys}
-    ref_dir = "/root/reference/config/model"
+    # key-for-key against the reference files as parsed (tests/golden/make_reference_samples.py)
+    refs = yaml.safe_load(open(os.path.join(ROOT, "tests", "golden", "reference_model_configs.yaml")))
+    assert len(refs) == len(top)
     for fn, keys in top.items():
         cfg = yaml.safe_load(open(os.path.join(ROOT, "config", "model", fn)))
         assert list(cfg.keys()) == keys, fn
-        if os.path.isdir(ref_dir):  # build container: key-for-key against the reference file
-            ref = yaml.safe_load(open(os.path.join(ref_dir, fn.replace("-b200", ""))))
-            assert list(cfg.keys()) == list(ref.keys()), fn
+        ref = refs[fn.replace("-b200", "")]
+        assert list(cfg.keys()) == list(ref.keys()), fn
 
-            def strip(node):  # compare everything except the swapped model-class targets
-                if isinstance(node, dict):
-                    return {k: ("<cls>" if k == "_target_" and str(v).startswith(("nabladft_b200.", "schnetpack.", "nablaDFT.")) else strip(v))
-                            for k, v in node.items()}
-                return [strip(v) for v in node] if isinstance(node, list) else node
+        def strip(node):  # compare everything except the swapped model-class targets
+            if isinstance(node, dict):
+                return {k: ("<cls>" if k == "_target_" and str(v).startswith(("nabladft_b200.", "schnetpack.", "nablaDFT.")) else strip(v))
+                        for k, v in node.items()}
+            return [strip(v) for v in node] if isinstance(node, list) else node
 
-            assert strip(cfg) == strip(ref), fn
+        assert strip(cfg) == strip(ref), fn
 
 
 def test_schnet_export_matches_oracle_and_state_dict_names():
